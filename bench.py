@@ -37,6 +37,11 @@ over ranks.
   strong    (N > 1) the same global B = 2^20 split over the N GPUs.
   other_configs  (N = 1) BASELINE.json configs[2..4]: device timing + binding pipe.
 
+--dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (float64):
+x, value, gradient and the progress arrays of a fixed, seeded sample of the batch
+(instance_index.npy names the instances) and the gathered done bitmap, so that two
+builds can be compared output for output on the same inputs.
+
 --impl reference times the reference's own CPU implementation of the path on the
 host cores: oracle/_ref (the reference's headers compiled against the Eigen-API
 shim) or the plain-C oracle port -- whichever is present; it says which.  The
@@ -62,6 +67,8 @@ SEED = 12345
 LOG2_B = 20
 HBM_FALLBACK_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md fallback
 METRIC = "batched L-BFGS instances/sec (Rosenbrock d=128)"
+DUMP_INSTANCES = 16384  # --dump-outputs: instances sampled from the batch
+DUMP_SEED = 2024
 
 
 def host_threads() -> int:
@@ -233,10 +240,30 @@ def parity_sample(x0, state, prog, n_samples: int, threads: int):
             "checker": "oracle/libcno_oracle.so (CPU restatement of the reference path)"}
 
 
+def dump_outputs(out_dir, state, prog, bitmap):
+    """Writes one step's returned arrays (see the module docstring) as float64 .npy files: 16 MiB each for the
+    sampled x and gradient, well under 64 MiB in all."""
+    import numpy as np
+    import torch
+    B = state.x.shape[0]
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(B, min(B, DUMP_INSTANCES), replace=False))
+    sel = torch.from_numpy(idx).to(state.x.device)
+    arrays = {"instance_index": idx, "x": state.x[sel], "value": state.value[sel], "gradient": state.gradient[sel],
+              "num_iterations": prog.num_iterations[sel], "status": prog.status[sel], "nfev": prog.nfev[sel],
+              "x_delta": prog.x_delta[sel], "f_delta": prog.f_delta[sel], "gradient_norm": prog.gradient_norm[sel],
+              "done_bitmap": bitmap}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if torch.is_tensor(a) else a
+        if name in ("num_iterations", "nfev", "done_bitmap"):
+            a = a.view(np.uint32)  # unsigned counters / bit words held in int32 tensors
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--log2-batch", type=int, default=LOG2_B, help="per-GPU batch = 2^this")
@@ -246,7 +273,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the strong-scaling and other-config records")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the arrays the last timed step returned (a seeded sample of the batch) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the device path's outputs (--impl b200)")
 
     if args.impl == "reference":
         return run_reference(args)
@@ -371,6 +404,8 @@ def main():
 
     # ---- parity: strided instances of the timed batch against the CPU oracle ----
     parity = parity_sample(x0, state, prog, 256, threads) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, state, prog, bitmap)
 
     # ---- e2e through the host-buffer C ABI call (wall clock around the call) ----
     e2e = None

@@ -1,6 +1,7 @@
 """Lbfgsb<F, 5> (solver/lbfgsb.h:44-538; SURVEY.md 8(f) rank 4) -- the device kernel csrc/cno_lbfgsb.cuh against the
-REFERENCE'S OWN header compiled from /root/reference on the Eigen-API shim (oracle/_ref: cno_ref_lbfgsb_minimize) and
-against the fixtures that build produced (tests/golden/lbfgsb_*.npz), bit for bit on every output array.
+REFERENCE'S OWN header compiled on the Eigen-API shim (oracle/_ref: cno_ref_lbfgsb_minimize; its recorded outputs for the
+same inputs, reference_outputs.py) and against the fixtures that build produced (tests/golden/lbfgsb_*.npz), bit for bit
+on every output array.
 CPU: the device source under the warp emulation (tests/emu).  GPU (-m gpu): the kernel through the C ABI
 (cno_lbfgsb_minimize) and the Python / C++ mirrors."""
 import ctypes as C
@@ -13,10 +14,10 @@ import pytest
 import torch
 
 from oracle import oracle_binding as ob
+import reference_outputs as ro
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 KEYS = ("num_iterations", "status", "nfev", "x", "value", "gradient", "x_delta", "f_delta", "gradient_norm")
-needs_ref = pytest.mark.skipif(not ob.ref_available(), reason="oracle/_ref not built")
 
 
 @pytest.fixture(scope="module")
@@ -71,20 +72,18 @@ def test_reference_verify_starts_reach_the_minimum():
     assert np.all(z["value"] < 1e-4) and np.all(np.abs(z["x"] - 1.0) < 1e-3)
 
 
-@needs_ref
 def test_emulated_lbfgsb_active_bounds_and_infeasible_start(emu):
     """A start outside the box is projected first (:145-150); the solution sits on the active faces with a non-zero
     gradient there and a small projected gradient."""
     x0 = ob.fill_uniform((3, 8), 0, 5, -3.0, 3.0)
     lo, hi = np.full(8, -0.5), np.full(8, 0.8)
     r = _emulated(emu, x0, lo, hi)
-    o = ob.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0, lo, hi)
+    o = ro.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0, lo, hi)
     for k in KEYS:
-        assert np.array_equal(r[k].view(np.uint8), o[k].view(np.uint8)), k
+        assert ro.equal(r[k], o[k]), k
     assert np.all(r["x"] <= 0.8) and np.all(r["x"] >= -0.5) and np.any(r["x"] == 0.8)
 
 
-@needs_ref
 def test_emulated_lbfgsb_m10_equals_reference_header(emu):
     """Lbfgsb<F, 10> (lbfgsb.h:44-45: m is a template parameter): the kernel with ten pairs (2k up to 20 lanes of the
     compact representation) == the reference's own Lbfgsb<F, 10>, bit for bit; it differs from m = 5."""
@@ -93,12 +92,11 @@ def test_emulated_lbfgsb_m10_equals_reference_header(emu):
     stop = ob.lbfgsb_stop()
     stop.num_iterations = 30  # (past ten iterations the history is full and wraps: both regimes are covered)
     r = _emulated(emu, x0, lo, hi, stop=stop, m=10)
-    o = ob.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0, lo, hi, stop=stop, m=10)
+    o = ro.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0, lo, hi, stop=stop, m=10)
     for k in KEYS:
-        assert np.array_equal(r[k].view(np.uint8), o[k].view(np.uint8)), k
-    o5 = ob.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0, lo, hi, stop=stop)
-    assert not np.array_equal(o5["num_iterations"], o["num_iterations"]) or \
-        not np.array_equal(o5["x"].view(np.uint64), o["x"].view(np.uint64))
+        assert ro.equal(r[k], o[k]), k
+    o5 = ro.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0, lo, hi, stop=stop)
+    assert not ro.equal(o5["num_iterations"], o["num_iterations"]) or not ro.equal(o5["x"], o["x"])
 
 
 # ---- GPU -----------------------------------------------------------------------------------------------------------
@@ -129,30 +127,28 @@ def test_gpu_lbfgsb_matches_reference_fixtures(path):
 
 
 @pytest.mark.gpu
-@needs_ref
 @pytest.mark.parametrize("d,B", [(8, 256), (37, 128), (64, 96), (128, 64)])
 def test_gpu_lbfgsb_bitwise_equals_reference_header(d, B):
     rng = np.random.default_rng(d)
     x0 = ob.fill_uniform((B, d), 0, 31 + d, -2.5, 2.5)
     lo = rng.uniform(-1.5, -0.2, (B, d))
     hi = lo + rng.uniform(0.3, 2.0, (B, d))
-    r, o = _gpu(x0, lo, hi), ob.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0, lo, hi)
+    r, o = _gpu(x0, lo, hi), ro.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0, lo, hi)
     for k in KEYS:
-        assert np.array_equal(r[k].view(np.uint8), o[k].view(np.uint8)), k
+        assert ro.equal(r[k], o[k]), k
     assert np.all(r["x"] >= lo) and np.all(r["x"] <= hi)
     # one shared box, and no box at all (the unbounded path: every coordinate free, no breakpoint visited)
-    r, o = _gpu(x0[:32], np.full(d, -0.5), np.full(d, 0.8)), ob.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0[:32], np.full(d, -0.5), np.full(d, 0.8))
+    r, o = _gpu(x0[:32], np.full(d, -0.5), np.full(d, 0.8)), ro.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0[:32], np.full(d, -0.5), np.full(d, 0.8))
     for k in KEYS:
-        assert np.array_equal(r[k].view(np.uint8), o[k].view(np.uint8)), k
+        assert ro.equal(r[k], o[k]), k
     stop = ob.lbfgsb_stop()
     stop.num_iterations = 80
-    r, o = _gpu(x0[:32], None, None, stop), ob.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0[:32], None, None, stop=stop)
+    r, o = _gpu(x0[:32], None, None, stop), ro.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0[:32], None, None, stop=stop)
     for k in KEYS:
-        assert np.array_equal(r[k].view(np.uint8), o[k].view(np.uint8)), k
+        assert ro.equal(r[k], o[k]), k
 
 
 @pytest.mark.gpu
-@needs_ref
 @pytest.mark.parametrize("d,B", [(8, 128), (37, 96), (128, 48)])
 def test_gpu_lbfgsb_m10_bitwise_equals_reference_header(d, B):
     """Lbfgsb<F, 10>: GPU == the reference's own Lbfgsb<F, 10> (oracle/_ref), per-instance boxes and unbounded."""
@@ -160,11 +156,11 @@ def test_gpu_lbfgsb_m10_bitwise_equals_reference_header(d, B):
     x0 = ob.fill_uniform((B, d), 0, 77 + d, -2.5, 2.5)
     lo = rng.uniform(-1.5, -0.2, (B, d))
     hi = lo + rng.uniform(0.3, 2.0, (B, d))
-    r, o = _gpu(x0, lo, hi, m=10), ob.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0, lo, hi, m=10)
+    r, o = _gpu(x0, lo, hi, m=10), ro.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0, lo, hi, m=10)
     for k in KEYS:
-        assert np.array_equal(r[k].view(np.uint8), o[k].view(np.uint8)), k
+        assert ro.equal(r[k], o[k]), k
     stop = ob.lbfgsb_stop()
     stop.num_iterations = 60
-    r, o = _gpu(x0[:24], None, None, stop, m=10), ob.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0[:24], None, None, stop=stop, m=10)
+    r, o = _gpu(x0[:24], None, None, stop, m=10), ro.ref_lbfgsb_minimize(ob.FN_ROSENBROCK, x0[:24], None, None, stop=stop, m=10)
     for k in KEYS:
-        assert np.array_equal(r[k].view(np.uint8), o[k].view(np.uint8)), k
+        assert ro.equal(r[k], o[k]), k

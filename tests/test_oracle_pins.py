@@ -3,9 +3,9 @@
      the 7 cstep KATs (src/test/cstep_test.cc:54-204), verify.cc Far/Near
      (src/test/verify.cc:23,129,168-173,187-188,192), the Dockerfile.test quadratic
      (:35-42) and the AL-test half-norm solve (augmented_lagrangian_test.cc:661-683);
-  2. bit for bit against oracle/_ref = the reference's own headers compiled from
-     /root/reference against the Eigen-API shim (when built), and against the
-     committed fixtures that build produced (always).
+  2. bit for bit against oracle/_ref = the reference's own headers compiled on the
+     Eigen-API shim: its recorded outputs for the same inputs (reference_outputs.py),
+     and the committed fixtures that build produced.
 """
 import glob
 import os
@@ -14,15 +14,16 @@ import numpy as np
 import pytest
 
 from oracle import oracle_binding as ob
+import reference_outputs as ro
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
-IMPLS = ["oracle"] + (["ref"] if ob.ref_available() else [])
+IMPLS = ["oracle", "ref"]
 
 
 # ---- src/test/cstep_test.cc -------------------------------------------------
 @pytest.mark.parametrize("impl", IMPLS)
 def test_cstep_case1_quadratic_model(impl):  # :54-72
-    io, brackt, info, ret = ob.cstep([0, 0, -1, 0, 0, 0, 3, 1.5, 2, 0, 10], 0, impl=impl)
+    io, brackt, info, ret = ro.cstep([0, 0, -1, 0, 0, 0, 3, 1.5, 2, 0, 10], 0, impl=impl)
     assert ret == 0 and info == 1 and brackt == 1
     assert abs(io[6] - 1.0) < 1e-12
     assert io[0] == 0.0 and io[3] == 3.0 and io[4] == 1.5 and io[5] == 2.0
@@ -30,7 +31,7 @@ def test_cstep_case1_quadratic_model(impl):  # :54-72
 
 @pytest.mark.parametrize("impl", IMPLS)
 def test_cstep_case2_sign_flip(impl):  # :81-100
-    io, brackt, info, ret = ob.cstep([0, 2, -2, 0, 0, 0, 3, 0.5, 1, 0, 10], 0, impl=impl)
+    io, brackt, info, ret = ro.cstep([0, 2, -2, 0, 0, 0, 3, 0.5, 1, 0, 10], 0, impl=impl)
     assert ret == 0 and info == 2 and brackt == 1
     assert abs(io[6] - 2.0) < 1e-12
     assert (io[0], io[1], io[2]) == (3.0, 0.5, 1.0)
@@ -39,7 +40,7 @@ def test_cstep_case2_sign_flip(impl):  # :81-100
 
 @pytest.mark.parametrize("impl", IMPLS)
 def test_cstep_case3_advance(impl):  # :109-127
-    io, brackt, info, ret = ob.cstep([0, 8, -4, 0, 0, 0, 1, 4.5, -3, 0, 20], 0, impl=impl)
+    io, brackt, info, ret = ro.cstep([0, 8, -4, 0, 0, 0, 1, 4.5, -3, 0, 20], 0, impl=impl)
     assert ret == 0 and info == 3 and brackt == 0
     assert 1.0 < io[6] <= 20.0
     assert (io[0], io[1], io[2]) == (1.0, 4.5, -3.0)
@@ -47,33 +48,32 @@ def test_cstep_case3_advance(impl):  # :109-127
 
 @pytest.mark.parametrize("impl", IMPLS)
 def test_cstep_case4_extrapolate(impl):  # :138-151
-    io, brackt, info, ret = ob.cstep([0, 5, -1, 0, 0, 0, 1, 3.99, -1.03, 0, 50], 0, impl=impl)
+    io, brackt, info, ret = ro.cstep([0, 5, -1, 0, 0, 0, 1, 3.99, -1.03, 0, 50], 0, impl=impl)
     assert ret == 0 and info == 4 and brackt == 0 and io[6] == 50.0
 
 
 @pytest.mark.parametrize("impl", IMPLS)
 def test_cstep_clamp(impl):  # :155-168
-    io, brackt, info, ret = ob.cstep([0, 0, -1, 0, 0, 0, 3, 1.5, 2, 0.1, 0.75], 0, impl=impl)
+    io, brackt, info, ret = ro.cstep([0, 0, -1, 0, 0, 0, 3, 1.5, 2, 0.1, 0.75], 0, impl=impl)
     assert ret == 0 and 0.1 <= io[6] <= 0.75
 
 
 @pytest.mark.parametrize("impl", IMPLS)
 def test_cstep_safeguard(impl):  # :175-191
-    io, brackt, info, ret = ob.cstep([0, 0, -1, 1, 0.5, 1.5, 0.99, 0.49, 1.4, 0, 2], 1, impl=impl)
+    io, brackt, info, ret = ro.cstep([0, 0, -1, 1, 0.5, 1.5, 0.99, 0.49, 1.4, 0, 2], 1, impl=impl)
     assert ret == 0 and info == 1 and brackt == 1
     assert 0.0 <= io[6] <= 0.66 + 1e-12
 
 
 @pytest.mark.parametrize("impl", IMPLS)
 def test_cstep_rejects_non_descent(impl):  # :196-204
-    io, brackt, info, ret = ob.cstep([0, 0, 1, 0, 0, 0, 1, 0.5, 0.5, 0, 10], 0, impl=impl)
+    io, brackt, info, ret = ro.cstep([0, 0, 1, 0, 0, 0, 1, 0.5, 0.5, 0, 10], 0, impl=impl)
     assert ret == -1
 
 
 def test_cstep_oracle_equals_reference_random():
-    if not ob.ref_available():
-        pytest.skip("oracle/_ref not built")
     rng = np.random.default_rng(7)
+    calls = []
     for _ in range(2000):
         stx, stp = sorted(rng.uniform(0, 4, 2))
         if stx == stp:
@@ -81,10 +81,10 @@ def test_cstep_oracle_equals_reference_random():
         io = [stx, rng.normal(), -abs(rng.normal()) - 1e-3, rng.uniform(0, 6), rng.normal(),
               rng.normal(), stp, rng.normal(), rng.normal(), 0.0, 50.0]
         br = int(rng.integers(0, 2))
-        a = ob.cstep(io, br, impl="oracle")
-        b = ob.cstep(io, br, impl="ref")
-        assert np.array_equal(np.array(a[0]).view(np.uint64), np.array(b[0]).view(np.uint64))
-        assert a[1:] == b[1:]
+        calls.append(((io, br), {}))
+    a = ro.stacked("cstep", [ob.cstep(*args) for args, _ in calls])
+    b = ro.sweep("cstep", calls)
+    assert ro.equal(a["io"], b["io"]) and ro.equal(a["flags"], b["flags"])
 
 
 # ---- src/test/verify.cc, Dockerfile.test, augmented_lagrangian_test.cc ------
@@ -99,7 +99,7 @@ def _rosen2(x):
 @pytest.mark.parametrize("solver", [ob.LBFGS, ob.BFGS, ob.NEWTON])
 @pytest.mark.parametrize("x0", [[15.0, 8.0], [-1.0, 2.0]])  # verify.cc:168-173
 def test_verify_cc_rosenbrock_far_near(impl, solver, x0):
-    r = ob.minimize(solver, ob.FN_ROSENBROCK, np.array([x0]), impl=impl)
+    r = ro.minimize(solver, ob.FN_ROSENBROCK, np.array([x0]), impl=impl)
     assert abs(_rosen2(r["x"][0])) < PRECISION  # verify.cc:129
     assert r["status"][0] != 1  # not IterationLimit
 
@@ -108,7 +108,7 @@ def test_verify_cc_rosenbrock_far_near(impl, solver, x0):
 @pytest.mark.parametrize("x0", [[15.0, 8.0], [-1.0, 2.0]])
 def test_verify_cc_gradient_descent_far_near(impl, x0):
     """SOLVER_SETUP_CONSERVATIVE(GradientDescent, RosenbrockGradient), verify.cc:185."""
-    r = ob.minimize(ob.GRADIENT_DESCENT, ob.FN_ROSENBROCK, np.array([x0]), impl=impl,
+    r = ro.minimize(ob.GRADIENT_DESCENT, ob.FN_ROSENBROCK, np.array([x0]), impl=impl,
                     stop=ob.conservative_stop())
     assert abs(_rosen2(r["x"][0])) < PRECISION
 
@@ -117,21 +117,21 @@ def test_verify_cc_gradient_descent_far_near(impl, x0):
 @pytest.mark.parametrize("x0", [[15.0, 8.0], [-1.0, 2.0]])
 def test_verify_cc_conjugated_gradient_descent_far_near(impl, x0):
     """SOLVER_SETUP(ConjugatedGradientDescent, RosenbrockGradient), verify.cc:186."""
-    r = ob.minimize(ob.CONJUGATED_GRADIENT_DESCENT, ob.FN_ROSENBROCK, np.array([x0]), impl=impl)
+    r = ro.minimize(ob.CONJUGATED_GRADIENT_DESCENT, ob.FN_ROSENBROCK, np.array([x0]), impl=impl)
     assert abs(_rosen2(r["x"][0])) < PRECISION
     assert r["status"][0] != 1
 
 
 @pytest.mark.parametrize("impl", IMPLS)
 def test_dockerfile_quadratic(impl):  # Dockerfile.test:35-42
-    r = ob.minimize(ob.LBFGS, ob.FN_DIAG_QUADRATIC, np.array([[-10.0, 2.0]]), impl=impl)
+    r = ro.minimize(ob.LBFGS, ob.FN_DIAG_QUADRATIC, np.array([[-10.0, 2.0]]), impl=impl)
     assert abs(r["x"][0, 0]) < 1e-4 and abs(r["x"][0, 1]) < 1e-4
     assert abs(r["value"][0] - 5.0) < 1e-4
 
 
 @pytest.mark.parametrize("impl", IMPLS)
 def test_al_test_half_norm(impl):  # augmented_lagrangian_test.cc:661-683 (inner solve)
-    r = ob.minimize(ob.LBFGS, ob.FN_HALF_SQUARED_NORM, np.array([[5.0, 5.0]]), impl=impl)
+    r = ro.minimize(ob.LBFGS, ob.FN_HALF_SQUARED_NORM, np.array([[5.0, 5.0]]), impl=impl)
     assert np.all(np.abs(r["x"][0]) < 1e-6)
 
 
@@ -152,7 +152,7 @@ KEYS = ("x", "value", "gradient", "num_iterations", "status", "nfev", "x_delta",
 
 
 def _same(a, b, keys=KEYS):
-    return all(np.array_equal(a[k].view(np.uint8), b[k].view(np.uint8)) for k in keys)
+    return all(ro.equal(a[k], b[k]) for k in keys)
 
 
 @pytest.mark.parametrize("dtype", [np.float64, np.float32])
@@ -161,12 +161,10 @@ def _same(a, b, keys=KEYS):
                                       (ob.BFGS, 2), (ob.BFGS, 32), (ob.BFGS, 37),
                                       (ob.NEWTON, 2), (ob.NEWTON, 8)])
 def test_oracle_equals_reference_headers(dtype, policy, solver, d):
-    if not ob.ref_available():
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
     B = 6 if d >= 64 else 16
     x0 = ob.fill_uniform((B, d), 1000 * d, 99, -2.0, 2.0, dtype)
     a = ob.minimize(solver, ob.FN_ROSENBROCK, x0, policy=policy, impl="oracle")
-    b = ob.minimize(solver, ob.FN_ROSENBROCK, x0, policy=policy, impl="ref")
+    b = ro.minimize(solver, ob.FN_ROSENBROCK, x0, policy=policy, impl="ref")
     assert _same(a, b)
 
 
@@ -193,22 +191,21 @@ def test_oracle_equals_reference_headers_under_random_progress_settings(solver, 
     solver -- iteration limits, x / f deltas with 1-3 allowed violations, absolute and relative thresholds, past windows
     0-8 -- through the C oracle and through the reference's own progress.h (oracle/_ref); every output equal bit for
     bit, and every solver's sweep ends in at least three different statuses."""
-    if not ob.ref_available():
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
     if solver == ob.CONJUGATED_GRADIENT_DESCENT and dtype == np.float32:
         pytest.skip("ConjugatedGradientDescent is fp64 only (the reference mixes double into ScalarType vectors)")
     rng = np.random.default_rng(1234 + 10 * solver + (dtype == np.float32))
     d, B = 8, 8
-    seen = set()
+    calls = []
     for k in range(40):
         stop = _random_stop(rng)
         if solver in (ob.GRADIENT_DESCENT, ob.CONJUGATED_GRADIENT_DESCENT):
             stop.num_iterations = min(stop.num_iterations, 60)
         x0 = ob.fill_uniform((B, d), 17 * k, 4321, -2.0, 2.0, dtype)
-        a = ob.minimize(solver, ob.FN_ROSENBROCK, x0, impl="oracle", stop=stop)
-        b = ob.minimize(solver, ob.FN_ROSENBROCK, x0, impl="ref", stop=stop)
-        assert _same(a, b), (k, [getattr(stop, f[0]) for f in ob.Stop._fields_])
-        seen.update(int(v) for v in a["status"])
+        calls.append(((solver, ob.FN_ROSENBROCK, x0), {"stop": stop}))
+    a = ro.stacked("minimize", [ob.minimize(*args, **kw) for args, kw in calls])
+    b = ro.sweep("minimize", calls)
+    assert _same(a, b), [k for k in KEYS if not ro.equal(a[k], b[k])]
+    seen = set(a["status"].ravel().tolist())
     assert len(seen) >= 3, seen
 
 
@@ -216,8 +213,6 @@ def test_fused_lu_oracle_equals_reference_headers():
     """CNO_POLICY_DMMA_LU: the oracle's lu_solve(fused = 1) == the reference's newton_descent.h / armijo.h /
     progress.h on the shim whose lu().solve() fuses every multiply-subtract under this policy; d = 64 (the shape
     the tensor-core kernel is built for), 12 and Rosenbrock d = 8; and the committed fixture."""
-    if not ob.ref_available():
-        pytest.skip("oracle/_ref not built")
     rng = np.random.default_rng(11)
     for d, B in ((64, 6), (12, 5)):
         M = rng.uniform(-1, 1, (B, d, d))
@@ -231,21 +226,19 @@ def test_fused_lu_oracle_equals_reference_headers():
         stop = ob.default_stop()
         stop.num_iterations = 6
         a = ob.minimize(ob.NEWTON, ob.FN_DENSE_QUADRATIC, x0, data=data, impl="oracle", policy=ob.POLICY_DMMA_LU, stop=stop)
-        b = ob.minimize(ob.NEWTON, ob.FN_DENSE_QUADRATIC, x0, data=data, impl="ref", policy=ob.POLICY_DMMA_LU, stop=stop)
+        b = ro.minimize(ob.NEWTON, ob.FN_DENSE_QUADRATIC, x0, data=data, impl="ref", policy=ob.POLICY_DMMA_LU, stop=stop)
         assert _same(a, b)
         c = ob.minimize(ob.NEWTON, ob.FN_DENSE_QUADRATIC, x0, data=data, impl="oracle", stop=stop)
         assert not np.array_equal(a["x"].view(np.uint64), c["x"].view(np.uint64))
     x0 = ob.fill_uniform((16, 8), 8000, 99, -2.0, 2.0)
     assert _same(ob.minimize(ob.NEWTON, ob.FN_ROSENBROCK, x0, policy=ob.POLICY_DMMA_LU, impl="oracle"),
-                 ob.minimize(ob.NEWTON, ob.FN_ROSENBROCK, x0, policy=ob.POLICY_DMMA_LU, impl="ref"))
+                 ro.minimize(ob.NEWTON, ob.FN_ROSENBROCK, x0, policy=ob.POLICY_DMMA_LU, impl="ref"))
 
 
 def test_condition_hessian_oracle_equals_reference_progress_update():
     """progress.condition_hessian (progress.h:203-210): the oracle's restatement == the value the reference's own
     Progress::Update leaves (oracle/_ref: H.norm() * H.inverse().norm() on the shim), fp64 (both LU policies), fp32,
     dense quadratics and the Rosenbrock Hessian; and the known answer for H = I."""
-    if not ob.ref_available():
-        pytest.skip("oracle/_ref not built")
     rng = np.random.default_rng(1)
     for d, B, dt in ((64, 4, np.float64), (12, 5, np.float64), (64, 3, np.float32)):
         M = rng.uniform(-1, 1, (B, d, d))
@@ -256,13 +249,12 @@ def test_condition_hessian_oracle_equals_reference_progress_update():
         x = rng.uniform(-2, 2, (B, d)).astype(dt)
         for pol in ((None, ob.POLICY_DMMA_LU) if dt == np.float64 else (None,)):
             a = ob.condition_hessian(ob.FN_DENSE_QUADRATIC, x, data=data, policy=pol)
-            r = ob.condition_hessian(ob.FN_DENSE_QUADRATIC, x, data=data, policy=pol, impl="ref")
-            assert np.array_equal(a.view(np.uint8), r.view(np.uint8))
+            r = ro.condition_hessian(ob.FN_DENSE_QUADRATIC, x, data=data, policy=pol, impl="ref")
+            assert ro.equal(a, r)
             truth = np.array([np.linalg.norm(A[i]) * np.linalg.norm(np.linalg.inv(A[i])) for i in range(B)])
             assert np.allclose(a, truth, rtol=1e-4 if dt == np.float32 else 1e-10)
     x = ob.fill_uniform((6, 8), 0, 3, -2.0, 2.0)
-    assert np.array_equal(ob.condition_hessian(ob.FN_ROSENBROCK, x).view(np.uint8),
-                          ob.condition_hessian(ob.FN_ROSENBROCK, x, impl="ref").view(np.uint8))
+    assert ro.equal(ob.condition_hessian(ob.FN_ROSENBROCK, x), ro.condition_hessian(ob.FN_ROSENBROCK, x, impl="ref"))
     assert np.allclose(ob.condition_hessian(ob.FN_HALF_SQUARED_NORM, x), 8.0, rtol=1e-15)  # ||I||_F ||I^-1||_F = d
 
 
@@ -282,19 +274,15 @@ def test_fused_lu_oracle_reproduces_committed_reference_fixture():
     (ob.CONJUGATED_GRADIENT_DESCENT, np.float64, 37)])
 def test_oracle_descent_solvers_equal_reference_headers(policy, solver, dtype, d):
     """gradient_descent.h / conjugated_gradient_descent.h / armijo.h:52-68 compiled from the reference."""
-    if not ob.ref_available():
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
     x0 = ob.fill_uniform((8, d), 77 * d, 5, -2.0, 2.0, dtype)
     stop = ob.default_stop()
     stop.num_iterations = 400  # bounded: these solvers crawl on Rosenbrock
     a = ob.minimize(solver, ob.FN_ROSENBROCK, x0, policy=policy, impl="oracle", stop=stop)
-    b = ob.minimize(solver, ob.FN_ROSENBROCK, x0, policy=policy, impl="ref", stop=stop)
+    b = ro.minimize(solver, ob.FN_ROSENBROCK, x0, policy=policy, impl="ref", stop=stop)
     assert _same(a, b)
 
 
 def test_oracle_equals_reference_dense_quadratic():
-    if not ob.ref_available():
-        pytest.skip("oracle/_ref not built")
     rng = np.random.default_rng(3)
     d, B = 12, 5
     M = rng.uniform(-1, 1, (B, d, d))
@@ -304,7 +292,7 @@ def test_oracle_equals_reference_dense_quadratic():
     x0 = rng.uniform(-2, 2, (B, d))
     for solver in (ob.LBFGS, ob.BFGS, ob.NEWTON):
         a = ob.minimize(solver, ob.FN_DENSE_QUADRATIC, x0, data=data, impl="oracle")
-        b = ob.minimize(solver, ob.FN_DENSE_QUADRATIC, x0, data=data, impl="ref")
+        b = ro.minimize(solver, ob.FN_DENSE_QUADRATIC, x0, data=data, impl="ref")
         assert _same(a, b)
         xs = np.linalg.solve(A, bvec[..., None])[..., 0]
         assert np.allclose(a["x"], xs, atol=1e-4)
@@ -417,9 +405,7 @@ def test_oracle_logistic_matches_closed_form():
 @pytest.mark.parametrize("d", [2, 8, 37, 128])
 def test_oracle_second_mode_lbfgs_equals_reference_headers(d):
     """Lbfgs<RosenbrockFull> (Second mode -> diagonal preconditioner, lbfgs.h:116-139)."""
-    if not ob.ref_available():
-        pytest.skip("oracle/_ref not built")
     x0 = ob.fill_uniform((8 if d < 100 else 2, d), 0, 5, -2.0, 2.0)  # the reference inverts H every iteration
     a = ob.minimize(ob.LBFGS, ob.FN_ROSENBROCK, x0, mode=2)
-    b = ob.minimize(ob.LBFGS, ob.FN_ROSENBROCK, x0, mode=2, impl="ref")
+    b = ro.minimize(ob.LBFGS, ob.FN_ROSENBROCK, x0, mode=2, impl="ref")
     assert _same(a, b, ("x", "value", "gradient", "num_iterations", "status", "nfev"))
